@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the reference's headline metric on its named configurations, one JSON line on rank 0.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload mel|cluster] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload mel|cluster] [--impl ours|reference] [--dump-outputs DIR]
 
 Main line (BASELINE.json configs[1], the configuration the metric is quoted on):
     log-mel of 1 h of synthetic 16 kHz mono audio, 25 ms / 10 ms frames, 512-point FFT, 80 mels -> [360 001 x 80].
@@ -18,6 +18,9 @@ Attached sub-objects, each with its own parity field:
     `c5`      configs[4]: 64 meetings x 5 000 x 256 SHARDED over the ranks (LPT), labels gathered over NCCL and hashed
               against goldens produced by the compiled reference (tests/golden/c5_meetings.json): `labels_equal_ref`.
     `streaming`: p50 / p99 latency of small `.prePadded` calls (the production callers' shape).
+--dump-outputs DIR: after the timed steps rank 0 writes what the last timed step computed, as DIR/<name>.npy: the log-mel
+rows of the headline path (a fixed sample of MEL_DUMP_ROWS frames, drawn with seed 0, float32) and the cluster labels
+(float64) and centroids (float64) of the 10 000 x 256 problem.  Inputs are seeded, so two builds compare output for output.
 With N > 1 (torchrun) units are independent: no data-path collective; NCCL carries the barrier, the MAX-reduction of
 times and the gather of labels / checksums.  Timing: barrier + device sync on both sides, MAX over ranks.
 
@@ -40,6 +43,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is written next to the sources
 
 MEL_SAMPLES = 57_600_000
 MEL_FRAMES = 360_001
@@ -50,6 +54,7 @@ AHC_BYTES = 8.0 * CLUSTER_D * CLUSTER_N * CLUSTER_N                       # 2.04
 C4_CLIPS, C4_SAMPLES = 512, 480_000
 C5_MEETINGS, C5_N = 64, 5_000
 MEL_TOL = 1e-4
+MEL_DUMP_ROWS = 65_536                                                    # 21 MB of the 115 MB output
 
 
 def measured_peaks():
@@ -297,7 +302,7 @@ def bench_mel(args, dist, clocks):
         out["roofline"]["frac"] = out["f64_transform"]["roofline_frac"]
         out["roofline"]["achieved"] = out["roofline"]["frac"] * peak
         out["roofline"]["kernel"] = "mel512_kernel<8, double>"
-    return out, audio, got32
+    return out, audio, got32, (got32 if diff <= MEL_TOL else got64)
 
 
 def bench_streaming(args):
@@ -324,10 +329,10 @@ def bench_streaming(args):
     return out
 
 
-def bench_cluster(args, dist, steps=None):
+def bench_cluster(args, dist):
     from fluidaudio_b200 import _lib, sharding, synth
     from fluidaudio_b200.clustering import OfflineClusterer
-    steps = steps or args.steps
+    steps = args.steps
     emb, _ = synth.speaker_embeddings(CLUSTER_N, CLUSTER_D, CLUSTER_K, sigma=0.02, seed=42 + dist.rank)
     rho, psi = synth.synthetic_plda(emb, CLUSTER_R)
     pin_e = _lib.PinnedArray(emb.shape, np.float32); pin_e.array[:] = emb
@@ -477,6 +482,19 @@ def bench_c5(args, dist):
             "golden": "tests/golden/c5_meetings.json (compiled reference fastcluster + oracle port of the Swift stages)"}
 
 
+def dump_outputs(out_dir, mel_rows, cluster_res):
+    """The last timed step's results as .npy files (float32 / float64): a seeded sample of the log-mel rows, and the
+    cluster labels and centroids."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"cluster_labels": np.asarray(cluster_res.labels, np.float64),
+              "cluster_centroids": np.asarray(cluster_res.centroids, np.float64)}
+    if mel_rows is not None:
+        rows = np.sort(np.random.default_rng(0).choice(MEL_FRAMES, MEL_DUMP_ROWS, replace=False))
+        arrays["mel_rows_sample"] = np.ascontiguousarray(mel_rows[rows], np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -486,6 +504,7 @@ def main():
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only-main", action="store_true", help="skip the c4 / c5 / streaming sub-objects (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -541,13 +560,12 @@ def main():
 
     got32 = None
     if args.workload == "mel":
-        line, audio, got32 = bench_mel(args, dist, clocks)
-        extra_steps = max(3, min(args.steps, 5))
-        cluster_line, cluster_data = bench_cluster(args, dist, steps=extra_steps)
+        line, audio, got32, mel_out = bench_mel(args, dist, clocks)
+        cluster_line, cluster_data = bench_cluster(args, dist)
         line["cluster"] = {k: cluster_line[k] for k in ("metric", "value", "unit", "ms_per_step", "e2e", "roofline", "stages_ms",
                                                          "gpu_launches", "config", "labels_equal_ref",
                                                          "labels_deterministic_all_ranks")}
-        line["cluster"]["steps"] = extra_steps
+        line["cluster"]["steps"] = args.steps
         if not args.only_main:
             line["c4"] = bench_c4(args, dist)
             line["c5"] = bench_c5(args, dist)
@@ -555,8 +573,10 @@ def main():
                 line["streaming"] = bench_streaming(args)
     else:
         line, cluster_data = bench_cluster(args, dist)
-        audio = None
+        audio = mel_out = None
     line["clocks"] = clocks.summary()
+    if args.dump_outputs and dist.is_root:
+        dump_outputs(args.dump_outputs, mel_out, cluster_data[3])
 
     os.sched_setaffinity(0, all_cpus)      # the CPU baseline may use every host core again
     if dist.is_root and world == 1 and not args.no_cpu_baseline:

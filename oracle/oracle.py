@@ -1,7 +1,9 @@
 """ORACLE — TEST INFRASTRUCTURE ONLY.  Not part of the shipped product path.
 
 ctypes front-end to ``liboracle.so`` (our CPU restatement, ``oracle_*.cpp``) and, when present, to
-``_ref/liboracle_fc.so`` (the unmodified reference ``FastClusterWrapper.cpp`` compiled by ``make ref``).
+``_ref/liboracle_fc.so`` (the unmodified reference ``FastClusterWrapper.cpp`` compiled by ``make ref``); where that was
+not built, the restatement stands in for it only where it reproduces the reference's results recorded in
+``tests/golden/ref_linkage.json``.
 Importers allowed: ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s cpu_baseline / ``--impl reference``.
 The product package ``fluidaudio_b200`` must never import this module (tests enforce it).
 
@@ -13,6 +15,8 @@ Pipeline glue restated here (pure Python, O(N)):
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 from dataclasses import dataclass
@@ -22,6 +26,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = os.path.join(_HERE, "liboracle.so")
 _REF = os.path.join(_HERE, "_ref", "liboracle_fc.so")
+_RECORDED = os.path.join(os.path.dirname(_HERE), "tests", "golden", "ref_linkage.json")
 _REFERENCE_ROOT = "/root/reference"
 
 _f32p = np.ctypeslib.ndpointer(np.float32, flags="C_CONTIGUOUS")
@@ -56,6 +61,7 @@ class VbxConfig(C.Structure):
 
 _lib = None
 _ref = None
+_recorded = None
 
 
 def lib():
@@ -327,16 +333,57 @@ def l2_normalize_rows(x: np.ndarray) -> np.ndarray:
     return out
 
 
-def centroid_linkage(x: np.ndarray, use_ref: bool = False):
-    """Returns (status, Z [(N-1) x 4]).  use_ref=True calls the compiled reference instead of the restatement."""
+def _linkage_key(x: np.ndarray) -> str:
+    return hashlib.sha256(np.asarray(x.shape, np.int64).tobytes() + x.tobytes()).hexdigest()[:32]
+
+
+def _linkage_record(status: int, z: np.ndarray) -> dict:
+    """What is kept of a reference result: its status and, when it succeeded, the SHA-256 of the dendrogram bytes."""
+    return {"status": int(status), "z_sha256": hashlib.sha256(z.tobytes()).hexdigest() if status == 0 else None}
+
+
+def reference_linkage(x: np.ndarray):
+    """The reference's (status, Z) for x.  Computed by the compiled reference where `make ref` built it; elsewhere the
+    restatement's result, accepted only if it reproduces the reference's status and dendrogram bytes (SHA-256) recorded for
+    the same input in tests/golden/ref_linkage.json (how to record new inputs: tests/golden/make_golden.py).  With
+    FA_ORACLE_RECORD_REF=<dir> every call to the compiled reference also stores its record under <dir>."""
+    global _recorded
     x = np.ascontiguousarray(x, np.float64)
+    key = _linkage_key(x)
+    if ref() is None:
+        if _recorded is None:
+            with open(_RECORDED) as f:
+                _recorded = json.load(f)
+        if key not in _recorded:
+            raise LookupError(f"no recorded reference result for this {x.shape} input (key {key}): record it with the "
+                              "compiled reference (tests/golden/make_golden.py)")
+        st, z = centroid_linkage(x)
+        if _linkage_record(st, z) != _recorded[key]:
+            raise AssertionError(f"the restatement differs from the reference's recorded result for this {x.shape} input "
+                                 f"(key {key})")
+        return st, z
     n, d = x.shape
     z = np.zeros((max(n - 1, 0), 4), np.float64)
     zp = z.ctypes.data if z.size else C.cast(C.create_string_buffer(8), C.c_void_p).value
+    st = int(ref().fastcluster_compute_centroid_linkage(x.ctypes.data, n, d, zp, z.size))
+    out_dir = os.environ.get("FA_ORACLE_RECORD_REF")
+    if out_dir:
+        os.makedirs(out_dir, exist_ok=True)
+        with open(os.path.join(out_dir, key + ".json"), "w") as f:
+            json.dump(_linkage_record(st, z), f)
+    return st, z
+
+
+def centroid_linkage(x: np.ndarray, use_ref: bool = False):
+    """Returns (status, Z [(N-1) x 4]).  use_ref=True gives the reference's result (reference_linkage) instead of the
+    restatement's."""
+    x = np.ascontiguousarray(x, np.float64)
     if use_ref:
-        st = ref().fastcluster_compute_centroid_linkage(x.ctypes.data, n, d, zp, z.size)
-    else:
-        st = lib().oracle_centroid_linkage(x.ctypes.data, n, d, zp, z.size)
+        return reference_linkage(x)
+    n, d = x.shape
+    z = np.zeros((max(n - 1, 0), 4), np.float64)
+    zp = z.ctypes.data if z.size else C.cast(C.create_string_buffer(8), C.c_void_p).value
+    st = lib().oracle_centroid_linkage(x.ctypes.data, n, d, zp, z.size)
     return int(st), z
 
 

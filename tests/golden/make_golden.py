@@ -9,10 +9,16 @@
               whose inputs are regenerated from seeds (fluidaudio_b200/synth.py) instead of being stored.
 * next_rows.npz  the rows either side of the hot path (SURVEY 8f): seeded K-Means runs, UnifiedMelExtractor and LS-EEND
               features from the oracle restatement (`python tests/golden/make_golden.py next` regenerates only these).
+* ref_linkage.json  the reference's status and dendrogram SHA-256 for every input on which the tests and smoke() ask for
+              its result (oracle.reference_linkage, keyed by a hash of the input bytes), so that those comparisons run
+              where the reference cannot be compiled.  Record them by running the whole suite (GPU tests included)
+              and smoke() with oracle/_ref built and FA_ORACLE_RECORD_REF=<dir>, then
+              `python tests/golden/make_golden.py ref_linkage <dir>`.
 * mel_*.npz   log-mel of the reference's own test signal (SortformerStreamingMelTests.swift:17-25 shape) from the
               oracle restatement: the reference has no golden mel values and no Swift toolchain exists here, so
               these pin the oracle against silent drift, not against Apple's vDSP.
 """
+import glob
 import hashlib
 import json
 import os
@@ -55,10 +61,23 @@ def next_rows():
     print("next_rows.npz written:", sorted(out))
 
 
+def pack_ref_linkage(src):
+    """Merges the reference records written under `src` into ref_linkage.json, keeping the entries already there."""
+    path = os.path.join(HERE, "ref_linkage.json")
+    records = json.load(open(path)) if os.path.exists(path) else {}
+    for rec in sorted(glob.glob(os.path.join(src, "*.json"))):
+        records[os.path.basename(rec)[:-5]] = json.load(open(rec))
+    with open(path, "w") as f:
+        f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(records[k])}" for k in sorted(records)) + "\n}\n")
+    print(f"{len(records)} reference records in {path}")
+
+
 def main():
     O.build()
     if len(sys.argv) > 1 and sys.argv[1] == "next":
         return next_rows()
+    if len(sys.argv) > 2 and sys.argv[1] == "ref_linkage":
+        return pack_ref_linkage(sys.argv[2])
     assert O.ref_available(), "oracle/_ref/liboracle_fc.so missing: run `make -C oracle ref` where /root/reference exists"
     rng = np.random.default_rng(2024)
     cases = {}

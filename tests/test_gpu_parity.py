@@ -447,7 +447,7 @@ def test_audio_to_mel_fused_pipeline(gpu_lib, oracle):
 
 # ================================================================================================ AHC
 def _ref_linkage(oracle, x):
-    return oracle.centroid_linkage(x, use_ref=oracle.ref_available())
+    return oracle.centroid_linkage(x, use_ref=True)
 
 
 def test_linkage_reproduces_reference_goldens_bit_exact(gpu_lib, golden_dir):
@@ -516,9 +516,9 @@ def test_linkage_float32_filter_is_bit_exact(gpu_lib, golden_dir, oracle):
         "from fluidaudio_b200 import synth\n"
         "e, _ = synth.speaker_embeddings(3000, 256, 4, seed=2); cases.append(O.l2_normalize_rows(e.astype(np.float64)))\n"
         "for x in cases:\n"
-        "    st, z = cl.centroid_linkage(x); st2, z2 = O.centroid_linkage(x, use_ref=O.ref_available()); ok = ok and st == st2 and np.array_equal(z, z2)\n"
+        "    st, z = cl.centroid_linkage(x); st2, z2 = O.centroid_linkage(x, use_ref=True); ok = ok and st == st2 and np.array_equal(z, z2)\n"
         "bad = rng.standard_normal((100, 8)); bad[50, 3] = np.nan\n"
-        "ok = ok and cl.centroid_linkage(bad)[0] == O.centroid_linkage(bad, use_ref=O.ref_available())[0] == 5\n"
+        "ok = ok and cl.centroid_linkage(bad)[0] == O.centroid_linkage(bad, use_ref=True)[0] == 5\n"
         "print('FILTER_OK' if ok else 'FILTER_BAD')" % (ROOT, golden_dir))
     for env in ({"FA_AHC_FILTER_MIN_N": "2"}, {"FA_AHC_FILTER_MIN_N": "0"}):
         out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, **env), capture_output=True, text=True, timeout=900)
@@ -627,7 +627,7 @@ def test_cluster_pipeline_labels_bit_exact(gpu_lib, oracle):
             emb[n - 1, 100] = np.inf
         rho, psi = synth.synthetic_plda(np.nan_to_num(emb, posinf=0.0))
         r = cl.OfflineClusterer(psi=psi).cluster(emb, rho)
-        o = oracle.diarize_cluster(emb, rho, psi, use_ref=oracle.ref_available())
+        o = oracle.diarize_cluster(emb, rho, psi, use_ref=True)
         assert np.array_equal(r.labels, o.labels), n
         assert np.array_equal(r.initial[o.training_indices], o.initial)
         assert r.info["training_count"] == o.training_indices.size
@@ -718,7 +718,7 @@ def test_constrained_pipeline_matches_oracle(gpu_lib, oracle):
         rho, psi = synth.synthetic_plda(emb)
         chunk = np.sort(rng.integers(0, n // 2, n)).astype(np.int32)        # ~2 local speakers per chunk
         r = cl.OfflineClusterer(psi=psi).cluster(emb, rho, chunk_indices=chunk)
-        o = oracle.diarize_cluster(emb, rho, psi, use_ref=oracle.ref_available(), chunk_indices=chunk)
+        o = oracle.diarize_cluster(emb, rho, psi, use_ref=True, chunk_indices=chunk)
         assert np.array_equal(r.labels, o.labels)
         plain = cl.OfflineClusterer(psi=psi).cluster(emb, rho).labels
         assert (r.labels != plain).any() or r.info["centroid_count"] == 1       # the constraint changes something
@@ -744,7 +744,7 @@ def test_export_replay_matches_oracle_and_file_labels(gpu_lib, oracle, tmp_path)
     for c in np.unique(chunk):                                                    # local speaker slots 0, 1, 2 ... per chunk
         idx = np.nonzero(chunk == c)[0]
         spk[idx] = np.arange(idx.size) % 3
-    o = oracle.diarize_cluster(emb, rho, psi, use_ref=oracle.ref_available(), chunk_indices=chunk)
+    o = oracle.diarize_cluster(emb, rho, psi, use_ref=True, chunk_indices=chunk)
     stored = np.where(o.labels >= 0, (o.labels + 3) % (o.labels.max() + 1), o.labels).astype(np.int32)   # renamed ids
     ex = EmbeddingExport(chunk, spk, (chunk * 10).astype(np.int32), (chunk * 10 + 9).astype(np.int32),
                          chunk * 0.17, chunk * 0.17 + 0.16, emb, rho, stored)
@@ -760,7 +760,7 @@ def test_export_replay_matches_oracle_and_file_labels(gpu_lib, oracle, tmp_path)
                                                          max(int(o.labels.max()) + 1, 1)))
     plain = cluster_prepared(prep, psi, constrained=False)
     assert np.array_equal(plain.result.labels,
-                          oracle.diarize_cluster(emb, rho, psi, use_ref=oracle.ref_available()).labels)
+                          oracle.diarize_cluster(emb, rho, psi, use_ref=True).labels)
 
 
 def test_mel_adapters_match_oracle(gpu_lib, oracle):
@@ -833,7 +833,7 @@ def test_speaker_count_constraints_pipeline_matches_oracle(gpu_lib, oracle):
         c = cfg.clustering
         for chunks in (None, chunk):
             r = cl.OfflineClusterer(cfg, psi=psi).cluster(emb, rho, chunk_indices=chunks)
-            o = oracle.diarize_cluster(emb, rho, psi, use_ref=oracle.ref_available(), chunk_indices=chunks,
+            o = oracle.diarize_cluster(emb, rho, psi, use_ref=True, chunk_indices=chunks,
                                        num_speakers=c.num_speakers, min_speakers=c.min_speakers, max_speakers=c.max_speakers)
             assert bool(r.info["was_adjusted"]) == o.was_adjusted and r.info["detected_clusters"] == o.detected_clusters
             assert np.array_equal(r.labels, o.labels), kw
@@ -862,7 +862,7 @@ def test_vbx_with_hundreds_and_thousands_of_speakers(gpu_lib, oracle):
     cfg = cl.OfflineDiarizerConfig()
     cfg.clustering.threshold = 0.2
     r = cl.OfflineClusterer(cfg, psi=psi).cluster(emb, rho)
-    o = oracle.diarize_cluster(emb, rho, psi, threshold=0.2, use_ref=oracle.ref_available())
+    o = oracle.diarize_cluster(emb, rho, psi, threshold=0.2, use_ref=True)
     assert r.info["initial_clusters"] == len(set(o.initial.tolist())) and r.info["initial_clusters"] > 200
     assert r.info["vbx_iterations"] == o.vbx.elbos.size and r.centroids.shape == o.centroids.shape
     assert np.abs(r.centroids - o.centroids).max() < 1e-9
@@ -906,7 +906,7 @@ def test_pipeline_odd_shapes_and_tiny_inputs(gpu_lib, oracle):
         rho, psi = synth.synthetic_plda(np.nan_to_num(emb, nan=0.0, posinf=0.0, neginf=0.0), min(128, d))
         for p in (psi, psi[:-1]):                                   # second pass: wrong length -> identity on both sides
             got = cl.OfflineClusterer(psi=p).cluster(emb, rho)
-            ref = oracle.diarize_cluster(emb, rho, p, use_ref=oracle.ref_available())
+            ref = oracle.diarize_cluster(emb, rho, p, use_ref=True)
             assert got.info["training_count"] == ref.training_indices.size
             assert np.array_equal(got.initial[got.initial >= 0], ref.initial)
             assert got.centroids.shape == ref.centroids.shape and np.abs(got.centroids - ref.centroids).max() < 1e-9
