@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(kWarps * 32, 2) mel512_kernel(const MelLaunch 
     };
     // time-major tile is contiguous in HBM: nf rows of n_mels floats; flat, fully coalesced copy out of otile
     auto copy_out = [&](float *dst, int total) {
-        if ((P.n_mels & 3) == 0) {   // rows are whole float4s and dst is 64-byte aligned (f0 is a multiple of 16)
+        if (P.vec_out) {   // rows are whole float4s and dst is 16-byte aligned (the unit's output is, and f0 is a multiple of 16)
             float4 *d4 = reinterpret_cast<float4 *>(dst);
             for (int q = tid; q < (total >> 2); q += kWarps * 32) {
                 const int e = 4 * q;
@@ -232,9 +232,11 @@ __global__ void __launch_bounds__(kWarps * 32, 2) mel512_kernel(const MelLaunch 
                 d4[q] = *reinterpret_cast<const float4 *>(otile + e + 4 * row);             // row stride n_mels + 4: one LDS.128
             }
         } else {
+            const int row_pad = ot_stride - P.n_mels;                        // 1, or 4 when a caller's output is not 16-byte aligned
             for (int idx = tid; idx < total; idx += kWarps * 32) {
-                const int fi = (int)__umulhi((unsigned)idx, P.inv_n_mels);   // idx / n_mels (exact for idx < 2^16)
-                dst[idx] = otile[idx + fi];                                  // padded row stride n_mels + 1
+                // idx / n_mels (exact for idx < 2^16); ceil(2^32 / 1) does not fit the 32-bit reciprocal
+                const int fi = P.n_mels == 1 ? idx : (int)__umulhi((unsigned)idx, P.inv_n_mels);
+                dst[idx] = otile[idx + fi * row_pad];                        // padded row stride n_mels + row_pad
             }
         }
     };
@@ -468,6 +470,23 @@ void build_filterbank(int n_fft, int n_mels, int sample_rate, std::vector<float>
 static constexpr int kWarpsPerCta = 8;
 static constexpr int kCtasPerSm = 2;
 
+// Dynamic shared memory of mel512_kernel (the layout at the top of the kernel) and the tile extents it is made of.
+static size_t mel512_smem_bytes(int hop, int n_mels, int fb_nnz, int n_slots, int *pt_len_out = nullptr,
+                                int *pt_cap_out = nullptr, int *raw_cap_out = nullptr, int *fb_cap_out = nullptr) {
+    const int pt_len = (kTileFrames - 1) * hop + kNfft;
+    const int pt_cap = (pt_len + 31) & ~31;
+    const int raw_cap = (pt_len + 1 + 3 + 3 + 31) & ~31;   // whole 128-byte lines: the pre-emphasised tile behind it stays line-aligned
+    const int fb_cap = (fb_nnz + 3) & ~3;
+    if (pt_len_out) *pt_len_out = pt_len;
+    if (pt_cap_out) *pt_cap_out = pt_cap;
+    if (raw_cap_out) *raw_cap_out = raw_cap;
+    if (fb_cap_out) *fb_cap_out = fb_cap;
+    return sizeof(float) * ((size_t)2 * raw_cap + pt_cap + 0 +
+                            (size_t)(kTileFrames / 2) * kPairStride + (size_t)kTileFrames * (n_mels + 4) + fb_cap) +
+           sizeof(cpxd) * (size_t)kWarpsPerCta * kFftPad + sizeof(int) * 4 * (size_t)n_slots + 8 +
+           2 * sizeof(uint64_t) + 3 * sizeof(TileInfo) + 16;
+}
+
 MelPlan::~MelPlan() { release(); }
 
 void MelPlan::release() {
@@ -521,7 +540,8 @@ int MelPlan::init(const MelConfig &c) {
                       cfg.n_fft, cfg.hop_length, cfg.win_length, cfg.n_mels);
         return FA_UNSUPPORTED;
     }
-    // the specialised kernel covers every in-repo caller's shape; anything else takes mel_generic_kernel
+    // the specialised kernel covers every in-repo caller's shape; anything else takes mel_generic_kernel (so do hops
+    // whose tile does not fit the specialised kernel's shared memory, decided below)
     generic = cfg.n_fft != kNfft || (cfg.hop_length & 1) || cfg.hop_length > 1024;
     const int n_fft = cfg.n_fft, bins = n_fft / 2 + 1;
     build_window(cfg.win_length, cfg.window_periodic != 0, window);
@@ -529,8 +549,8 @@ int MelPlan::init(const MelConfig &c) {
 
     // banded filterbank: per mel the contiguous range of non-zero bins, widened with explicit zero weights to whole
     // bin quads.  Weights are stored times 1/4 because the kernel's power tile holds 4|X|^2 (mel_core.cuh).
-    std::vector<float> w;
     std::vector<int> lo(cfg.n_mels), hi(cfg.n_mels), off(cfg.n_mels);
+    int nnz = 0;
     for (int m = 0; m < cfg.n_mels; ++m) {
         int a = bins, b = 0;
         for (int k = 0; k < bins; ++k)
@@ -543,15 +563,10 @@ int MelPlan::init(const MelConfig &c) {
         b = (b + 3) & ~3;              // may reach 260 > 257: the tile's pad columns are zero, so are these weights
         lo[m] = a;
         hi[m] = b;
-        off[m] = (int)w.size();        // a multiple of four: 16-byte aligned weight quads
-        // packed in the order the kernel finds the bins in its power tile: mel512_kernel swizzles inside each bin quad
-        // (pow_pos, mel_core.cuh), the any-nFFT kernel keeps the natural order
-        for (int k = a; k < b; ++k) {
-            const int src = generic ? k : ((k & ~3) | ((k & 3) ^ ((k >> 4) & 3)));   // position k holds bin src: pow_pos is an involution
-            w.push_back(src < bins ? 0.25f * filterbank[(size_t)m * bins + src] : 0.0f);
-        }
+        off[m] = nnz;                  // a multiple of four: 16-byte aligned weight quads
+        nnz += b - a;
     }
-    fb_nnz = (int)w.size();
+    fb_nnz = nnz;
     // filterbank-stage schedule of mel512_kernel: groups of four consecutive filters, dealt to the 8 warps longest first
     // (cost = widest band of the group, in quads); slot = (iteration * 8 + warp) * 4 + member
     std::vector<int4> slots;
@@ -599,6 +614,21 @@ int MelPlan::init(const MelConfig &c) {
         fa::set_error("fluidaudio_b200 requires an sm_100a device, found sm_%d%d", prop.major, prop.minor);
         return FA_NO_DEVICE;
     }
+    // mel512_kernel stages 15 hops + 512 samples three times (two raw buffers + the pre-emphasised tile): long even hops
+    // do not fit the per-CTA opt-in limit (on B200 from hop ~890 at 80 mels, ~680 at 512 mels) and take the any-nFFT
+    // kernel, which computes the same values
+    if (!generic && mel512_smem_bytes(cfg.hop_length, cfg.n_mels, fb_nnz, n_slots) > (size_t)prop.sharedMemPerBlockOptin)
+        generic = true;
+
+    // weights packed in the order the kernel finds the bins in its power tile: mel512_kernel swizzles inside each bin
+    // quad (pow_pos, mel_core.cuh), the any-nFFT kernel keeps the natural order
+    std::vector<float> w;
+    w.reserve(fb_nnz);
+    for (int m = 0; m < cfg.n_mels; ++m)
+        for (int k = lo[m]; k < hi[m]; ++k) {
+            const int src = generic ? k : ((k & ~3) | ((k & 3) ^ ((k >> 4) & 3)));   // position k holds bin src: pow_pos is an involution
+            w.push_back(src < bins ? 0.25f * filterbank[(size_t)m * bins + src] : 0.0f);
+        }
 
     std::vector<float> win_tab(n_fft, 0.0f);
     std::vector<uint8_t> in_tab(n_fft, 0);
@@ -670,19 +700,7 @@ int MelPlan::init(const MelConfig &c) {
         FA_CUDA_TRY(cudaFuncSetAttribute(mel_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
         return FA_OK;
     }
-    pt_len = (kTileFrames - 1) * cfg.hop_length + kNfft;
-    pt_cap = (pt_len + 31) & ~31;
-    raw_cap = (pt_len + 1 + 3 + 3 + 31) & ~31;   // whole 128-byte lines: the pre-emphasised tile behind it stays line-aligned
-    fb_cap = (fb_nnz + 3) & ~3;
-    smem_bytes = sizeof(float) * ((size_t)2 * raw_cap + pt_cap + 0 +
-                                  (size_t)(kTileFrames / 2) * kPairStride + (size_t)kTileFrames * (cfg.n_mels + 4) + fb_cap) +
-                 sizeof(cpxd) * (size_t)kWarpsPerCta * kFftPad + sizeof(int) * 4 * (size_t)n_slots + 8 +
-                 2 * sizeof(uint64_t) + 3 * sizeof(TileInfo) + 16;
-    if (smem_bytes > (size_t)prop.sharedMemPerBlockOptin) {
-        fa::set_error("mel config needs %zu bytes of shared memory per CTA, device allows %zu", smem_bytes,
-                      (size_t)prop.sharedMemPerBlockOptin);
-        return FA_UNSUPPORTED;
-    }
+    smem_bytes = mel512_smem_bytes(cfg.hop_length, cfg.n_mels, fb_nnz, n_slots, &pt_len, &pt_cap, &raw_cap, &fb_cap);
     FA_CUDA_TRY(cudaFuncSetAttribute(mel512_kernel<kWarpsPerCta, double, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
     FA_CUDA_TRY(cudaFuncSetAttribute(mel512_kernel<kWarpsPerCta, double, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
     FA_CUDA_TRY(cudaFuncSetAttribute(mel512_kernel<kWarpsPerCta, f32x2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
@@ -755,6 +773,10 @@ int MelPlan::launch(const float *d_audio_base, float *d_out_base, int first, int
     P.log_floor = cfg.log_floor;
     P.log_clamped = cfg.log_floor_mode;
     P.ot_stride = (cfg.n_mels & 3) == 0 ? cfg.n_mels + 4 : cfg.n_mels + 1;
+    // float4 row stores need a 16-byte aligned output: a caller's device pointer, batch output offsets or pinned view may
+    // not be (the units' descriptors are still in h_units)
+    P.vec_out = (cfg.n_mels & 3) == 0 && (reinterpret_cast<uintptr_t>(d_out_base) & 15) == 0;
+    for (int u = first; u < first + count && P.vec_out; ++u) P.vec_out = (h_units[u].out_off & 3) == 0;
     P.log_normal = cfg.log_floor >= 1e-37f ? 1 : 0;   // mel energies are >= 0: log's argument is then never a denormal
     P.layout = layout;
     P.lane_tab = d_lane_tab[mode == 2 ? 1 : 0][precision == 1 ? 1 : 0];
@@ -776,7 +798,7 @@ int MelPlan::launch(const float *d_audio_base, float *d_out_base, int first, int
         const int off_w = mode == 2 ? 0 : (cfg.n_fft - cfg.win_length) / 2;
         P.mid_full = (off_w <= 64 && off_w + cfg.win_length >= 448) ? 1 : 0;
     }
-    P.inv_n_mels = (unsigned)((0x100000000ull + (unsigned)cfg.n_mels - 1) / (unsigned)cfg.n_mels);
+    P.inv_n_mels = (unsigned)((0x100000000ull + (unsigned)cfg.n_mels - 1) / (unsigned)cfg.n_mels);   // 0 for n_mels == 1
     if (generic) {
         GenericParams G{cfg.n_fft, generic_log2n, cfg.n_fft / 2 + 1, generic_prow, reinterpret_cast<const cpxd *>(d_generic_tw),
                         generic_warps};

@@ -51,6 +51,7 @@ struct MelLaunch {
     float log_floor;
     int log_clamped;
     int ot_stride;      // floats per row of the staged output tile: n_mels + 4 (16-byte aligned rows) or n_mels + 1
+    int vec_out;        // time-major copy-out in float4 stores: n_mels % 4 == 0 and every unit's output 16-byte aligned
     int log_normal;     // log_floor is a normal float: the denormal handling of the device log can be skipped
     int layout;         // 0 time-major [T x nMels], 1 mel-major [nMels x stride]
     const void *lane_tab;   // [32] LaneTables<V> of the launch's window placement and precision (mel_core.cuh)
@@ -66,7 +67,7 @@ struct MelLaunch {
     int pt_len, pt_cap, raw_cap;
     int use_tma;
     int mid_full;          // window covers buffer positions [64, 448): pass 1 skips the in-window select for slots 1..6
-    unsigned inv_n_mels;   // ceil(2^32 / n_mels): idx / n_mels == umulhi(idx, inv) for idx < 2^16
+    unsigned inv_n_mels;   // ceil(2^32 / n_mels): idx / n_mels == umulhi(idx, inv) for idx < 2^16 (n_mels > 1)
     int inline_unit;       // single-unit launch: the descriptor travels in the kernel parameters (unit0), units is not read
     MelUnit unit0;
 };

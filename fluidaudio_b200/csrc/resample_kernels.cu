@@ -162,24 +162,28 @@ __global__ void __launch_bounds__(256) linear_kernel(Source s, double ratio, flo
 // Kaiser-windowed-sinc polyphase.  One CTA = 256 consecutive outputs; their input span (mixed down, widened) is staged
 // in shared memory once, every thread then runs its 2H-tap dot product out of shared memory: coefficients as 16-byte
 // loads through the read-only path (a single row when L == 1, i.e. integer decimation: every lane reads the same
-// address), four independent accumulators, 32-bit index arithmetic relative to one 64-bit division per CTA.
+// address), four independent accumulators, index arithmetic of type U relative to one 64-bit division per CTA.
+// A thread's phase numerator is base_ph + threadIdx.x * M < L + 255 M.  Integer rates keep that below 2^32 (U = unsigned,
+// 32-bit division); rates on the 1/1000 Hz grid do not (44100.001 Hz -> 16 kHz: L = 16 000 000, M = 44 100 001, and
+// 255 M ~ 1.1e10), so those take U = unsigned long long (see sinc_needs_64bit).
+template <typename U>
 __global__ void __launch_bounds__(256)
 sinc_kernel(Source s, long long L, long long M, int half, int phases, int exact, int row_stride,
             const float *__restrict__ tab, float *out, long long o_begin, long long o_end) {
     extern __shared__ float xs[];
     __shared__ long long base_n0;
-    __shared__ unsigned base_ph;
+    __shared__ U base_ph;
     const long long i0 = o_begin + (long long)blockIdx.x * 256;
     if (threadIdx.x == 0) {
         const long long num = i0 * M;
         base_n0 = num / L;
-        base_ph = (unsigned)(num - base_n0 * L);
+        base_ph = (U)(num - base_n0 * L);
     }
     __syncthreads();
-    const unsigned uL = (unsigned)L, uM = (unsigned)M;   // L, M < 2^22 (rates on a 1/1000 Hz grid): 255 * M + L < 2^31
+    const U uL = (U)L, uM = (U)M;
     const int last = (int)(min(i0 + 255, o_end - 1) - i0);
     const long long n_lo = base_n0 - half + 1;
-    const int span = (int)((base_ph + (unsigned)last * uM) / uL) + 2 * half;
+    const int span = (int)((base_ph + (U)last * uM) / uL) + 2 * half;
     for (int j = threadIdx.x; j < span + 4; j += 256) {
         const long long n = n_lo + j;
         xs[j] = (j < span && n >= 0 && n < s.frames) ? mono_at(s, n) : 0.0f;
@@ -187,8 +191,8 @@ sinc_kernel(Source s, long long L, long long M, int half, int phases, int exact,
     __syncthreads();
     const long long i = i0 + threadIdx.x;
     if (i >= o_end) return;
-    const unsigned t = base_ph + threadIdx.x * uM;
-    const unsigned dn = t / uL, ph = t - dn * uL;
+    const U t = base_ph + (U)threadIdx.x * uM;
+    const U dn = t / uL, ph = t - dn * uL;
     const float *x = xs + dn;          // input n0 - H + 1 + k sits at xs[dn + k]
     const int nq = row_stride >> 2;
     float a0 = 0.0f, a1 = 0.0f, a2 = 0.0f, a3 = 0.0f;
@@ -219,6 +223,9 @@ sinc_kernel(Source s, long long L, long long M, int half, int phases, int exact,
     out[i] = (a0 + a1) + (a2 + a3);
 }
 
+// L + 255 M (the largest phase numerator of a CTA, see sinc_kernel) does not fit 32 bits
+static bool sinc_needs_64bit(const Design &d) { return (unsigned long long)d.L + 255ull * (unsigned long long)d.M > 0xffffffffull; }
+
 int launch_convert(const void *d_pcm, long long frames, const AudioFormat &f, const Design &d, const float *d_tab,
                    float *d_out, long long o_begin, long long o_end, cudaStream_t stream, long long *launches) {
     if (o_end <= o_begin) return FA_OK;
@@ -230,10 +237,11 @@ int launch_convert(const void *d_pcm, long long frames, const AudioFormat &f, co
         linear_kernel<<<grid, 256, 0, stream>>>(s, f.in_rate / f.out_rate, d_out, o_begin, o_end);
     } else {
         const size_t smem = sizeof(float) * (size_t)((255 * d.M) / d.L + d.taps + 12);
+        auto *kernel = sinc_needs_64bit(d) ? sinc_kernel<unsigned long long> : sinc_kernel<unsigned>;
         if (smem > 48 * 1024)
-            FA_CUDA_TRY(cudaFuncSetAttribute(sinc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        sinc_kernel<<<grid, 256, smem, stream>>>(s, d.L, d.M, d.half, d.phases, d.exact ? 1 : 0, d.row_stride, d_tab, d_out,
-                                                 o_begin, o_end);
+            FA_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kernel<<<grid, 256, smem, stream>>>(s, d.L, d.M, d.half, d.phases, d.exact ? 1 : 0, d.row_stride, d_tab, d_out,
+                                            o_begin, o_end);
     }
     FA_CUDA_TRY(cudaGetLastError());
     if (launches) ++*launches;

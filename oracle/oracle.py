@@ -270,12 +270,20 @@ def resample_output_count(frames: int, in_rate: float, out_rate: float) -> int:
     return int(frames) if in_rate == out_rate else int(float(frames) / (in_rate / out_rate))
 
 
+def rational_ratio(in_rate: float, out_rate: float):
+    """out/in = L/M in lowest terms, reduced as the library does (resample_kernels.cu rational_ratio): integer rates as
+    they are, otherwise both rates on a 1/1000 Hz grid (rounded to the nearest grid point), then divided by their gcd."""
+    from math import floor, gcd
+    whole = lambda r: abs(r - round(r)) <= 1e-9
+    scale = 1 if whole(in_rate) and whole(out_rate) else 1000
+    a, b = int(floor(out_rate * scale + 0.5)), int(floor(in_rate * scale + 0.5))
+    g = gcd(a, b)
+    return a // g, b // g
+
+
 def sinc_design(in_rate: float, out_rate: float):
     """Returns (L, M, half, fc): out/in = L/M, half = taps / 2, fc relative to the input Nyquist."""
-    from math import gcd
-    a, b = int(round(out_rate)), int(round(in_rate))
-    g = gcd(a, b)
-    L, M = a // g, b // g
+    L, M = rational_ratio(in_rate, out_rate)
     lower = min(1.0, L / M)
     return L, M, int(np.ceil(SINC_ZEROS / lower)), lower * SINC_ROLLOFF
 
@@ -301,27 +309,40 @@ def mixdown(pcm: np.ndarray) -> np.ndarray:
     return s if x.shape[0] == 1 else (s * np.float32(1.0 / np.float32(x.shape[0]))).astype(np.float32)
 
 
-def sinc_resample(mono: np.ndarray, in_rate: float, out_rate: float) -> np.ndarray:
+def sinc_resample(mono: np.ndarray, in_rate: float, out_rate: float, first: int = 0, count=None) -> np.ndarray:
     """float64 evaluation of the documented polyphase filter on a mono float32 signal (rows normalised to unit DC gain
-    exactly as the library's float32 table is, so the only difference left is float32 rounding of taps and sums)."""
+    exactly as the library's float32 table is, so the only difference left is float32 rounding of taps and sums).
+    Evaluates outputs [first, first + count) of the whole signal's resampling (default: all of them), each at its exact
+    phase (i * M) mod L, so a window at the far end of a long signal costs what a window at its start does."""
     x = np.asarray(mono, np.float32).astype(np.float64)
     n = x.size
-    count = resample_output_count(n, in_rate, out_rate)
+    total = resample_output_count(n, in_rate, out_rate)
+    count = total - first if count is None else int(count)
+    if first < 0 or count < 0 or first + count > total:
+        raise ValueError(f"outputs [{first}, {first + count}) outside [0, {total})")
     if in_rate == out_rate:
-        return x.astype(np.float32)
+        return x[first:first + count].astype(np.float32)
     L, M, half, fc = sinc_design(in_rate, out_rate)
-    xp = np.concatenate([np.zeros(half), x, np.zeros(half + 2)])
-    out = np.zeros(count)
     k = np.arange(-half + 1, half + 1)
-    i = np.arange(count, dtype=np.int64)
-    n0 = (i * M) // L
-    ph = (i * M) % L
-    for p in np.unique(ph):
-        sel = np.nonzero(ph == p)[0]
-        row = _sinc_kernel(k - p / L, half, fc)
-        row = row / row.sum()
-        idx = n0[sel][:, None] + k[None, :] + half
-        out[sel] = (xp[idx] * row[None, :]).sum(axis=1)
+    rows_of = None
+    if L <= 4096:                   # few distinct phases: one normalised row per phase, shared by the outputs
+        table = _sinc_kernel(k[None, :] - np.arange(L)[:, None] / L, half, fc)
+        table /= table.sum(axis=1, keepdims=True)
+        rows_of = lambda ph: table[ph]
+    out = np.zeros(count)
+    block = 4096
+    for s in range(0, count, block):
+        i = np.arange(first + s, first + min(s + block, count), dtype=np.int64)
+        num = i * M                 # < 2^63 for any signal a test can hold
+        n0, ph = num // L, num % L
+        if rows_of is not None:
+            rows = rows_of(ph)
+        else:
+            rows = _sinc_kernel(k[None, :] - ph[:, None] / L, half, fc)
+            rows /= rows.sum(axis=1, keepdims=True)
+        idx = n0[:, None] + k[None, :]
+        xs = np.where((idx >= 0) & (idx < n), x[np.clip(idx, 0, max(n - 1, 0))], 0.0)
+        out[s:s + i.size] = (xs * rows).sum(axis=1)
     return out.astype(np.float32)
 
 
