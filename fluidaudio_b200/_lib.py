@@ -74,7 +74,7 @@ EXPORTED_SYMBOLS = [
     "fa_resample_output_count", "fa_audio_resample", "fa_audio_to_mel",
     "fa_linear_resample", "fa_l2_normalize_rows", "fa_ahc_cluster", "fa_dendrogram_cut", "fa_vbx_default_config",
     "fa_vbx_refine", "fa_compute_centroids", "fa_assign_embeddings", "fa_cluster_default_config",
-    "fa_diarize_cluster", "fa_diarize_cluster_batch", "fa_diarize_cluster_batch_chunks", "fa_ahc_last_stage_ms", "fa_diarize_cluster_chunks",
+    "fa_diarize_cluster", "fa_diarize_cluster_batch", "fa_diarize_cluster_batch_chunks", "fa_ahc_last_stage_ms", "fa_ahc_last_placement", "fa_diarize_cluster_chunks",
     "fa_hungarian_solve", "fa_max_score_assignment", "fa_constrained_assign", "fa_build_chunk_assignments",
     "fa_export_shape", "fa_export_read", "fa_export_write", "fa_kmeans_cluster", "fa_speaker_constraints_resolve",
     "fa_reconstruct_default_config", "fa_build_segments", "fa_build_speaker_database",
@@ -169,6 +169,8 @@ def load():
     L.fa_export_write.argtypes = [C.c_char_p, sz, sz, sz, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.fa_ahc_last_stage_ms.argtypes = [vp]
     L.fa_ahc_last_stage_ms.restype = None
+    L.fa_ahc_last_placement.argtypes = [vp]
+    L.fa_ahc_last_placement.restype = None
     L.fastcluster_compute_centroid_linkage.argtypes = [vp, sz, sz, vp, sz]
     L.fastcluster_compute_centroid_linkage.restype = C.c_int
     _lib = L

@@ -1179,6 +1179,8 @@ int launch_widen_rows(const float *d_in, double *d_out, long long count, cudaStr
 // ------------------------------------------------------------------------------------------------ host solver
 thread_local float g_last_ms[4] = {0, 0, 0, 0};
 const float *last_stage_ms() { return g_last_ms; }
+thread_local int g_placement[6] = {0, 0, 0, 0, 0, 0};
+const int *last_placement() { return g_placement; }
 
 Solver::~Solver() { release(); }
 
@@ -1380,6 +1382,12 @@ int Solver::linkage_device(const double *d_rows, int N, int D, double *Z) {
         }
     }
     const size_t smem = std::max(worker_smem, level ? master_smem_bytes(N, level) : (size_t)0);
+    g_placement[0] = level;
+    g_placement[1] = resident ? 1 : 0;
+    g_placement[2] = workers;
+    g_placement[3] = slots_per_cta;
+    g_placement[4] = kInitExact;
+    g_placement[5] = num_sms;
     int st = ensure_pool(N, D);
     if (st != FA_OK) return st;
     const Layout L = make_layout(N, D, Ns, max_workers);
@@ -1488,10 +1496,13 @@ int Solver::linkage_device(const double *d_rows, int N, int D, double *Z) {
             const int nt2 = (N + kGT - 1) / kGT;
             ahc_filter_tile128_kernel<<<(unsigned)((long long)nt2 * (nt2 + 1) / 2), 256, 0, stream>>>(N, D, Ns, F);
         }
-        if (!(hk.filter_impl & 2) && F.tmin && (size_t)8 * D * sizeof(float) <= 48 * 1024)
+        if (!(hk.filter_impl & 2) && F.tmin && (size_t)8 * D * sizeof(float) <= 48 * 1024) {
             ahc_filter_rows_kernel<<<(N + 7) / 8, 256, (size_t)8 * D * sizeof(float), stream>>>(N, D, Ns, F);
-        else
+            g_placement[4] = kInitFilterRows;
+        } else {
             ahc_filter_tile_kernel<true><<<tiles, 256, 0, stream>>>(N, D, Ns, F);
+            g_placement[4] = kInitFilterTiles;
+        }
         const unsigned cgrid = (unsigned)((F.cap + 255) / 256);
         ahc_filter_exact_kernel<<<cgrid, 256, 0, stream>>>(P.cols, D, Ns, F);
         ahc_filter_argmin_kernel<<<cgrid, 256, 0, stream>>>(F);
@@ -1501,6 +1512,7 @@ int Solver::linkage_device(const double *d_rows, int N, int D, double *Z) {
         FA_CUDA_TRY(cudaMemcpyAsync(h_fc, F.counters, 3 * sizeof(int), cudaMemcpyDeviceToHost, stream));
         FA_CUDA_TRY(cudaStreamSynchronize(stream));
         if (h_fc[1] || h_fc[2]) {   // non-finite / huge input, or more candidates than the list holds: the exact pass decides
+            g_placement[4] = kInitFilterFellBack;
             const int st2 = exact_init();
             if (st2 != FA_OK) return st2;
         }

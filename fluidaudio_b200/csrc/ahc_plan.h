@@ -88,6 +88,9 @@ struct Solver {
 // [0] initial nearest-neighbour kernels, [1] heapify + copies, [2] merge kernel, [3] total (ms) of the calling
 // thread's most recent linkage
 const float *last_stage_ms();
+// placement of the calling thread's most recent linkage (layout: fa_ahc_last_placement in fluidaudio_b200.h)
+enum { kInitExact = 0, kInitFilterRows = 1, kInitFilterTiles = 2, kInitFilterFellBack = 3 };
+const int *last_placement();
 
 // Standalone kernels used by the clustering pipeline
 int launch_normalize_rows(const double *d_in, double *d_out, int rows, int dim, cudaStream_t s);

@@ -988,6 +988,12 @@ FA_API void fa_ahc_last_stage_ms(float *out4) {
     for (int q = 0; q < 4; ++q) out4[q] = m[q];
 }
 
+FA_API void fa_ahc_last_placement(int32_t *out6) {
+    if (!out6) return;
+    const int *p = ahc::last_placement();
+    for (int q = 0; q < 6; ++q) out6[q] = p[q];
+}
+
 FA_API fa_status fa_l2_normalize_rows(const double *x, size_t rows, size_t dim, double *out) {
     if (!x || !out) return FA_STATUS_INVALID_ARGUMENT;
     if (rows == 0 || dim == 0) return FA_STATUS_OK;

@@ -208,6 +208,17 @@ fa_status fa_ahc_cluster(const double *features, size_t count, size_t dim, doubl
  * [2] persistent merge kernel, [3] total (ms).  Diagnostics only. */
 void fa_ahc_last_stage_ms(float *out4);
 
+/* Placement the calling thread's most recent linkage ran with, as six values:
+ *   [0] master level: 3 = heap, nearest neighbours and slot table in shared memory, 2 = heap and nearest neighbours,
+ *       1 = heap only (all three with 16-bit heap indices), 0 = all in global memory (32-bit heap indices)
+ *   [1] 1 = node vectors resident in the workers' shared memory, 0 = streamed from global memory
+ *   [2] worker CTAs   [3] node slots per worker CTA (resident only, else 0)
+ *   [4] initial nearest-neighbour pass: 0 = exact, 1 = float32 filter with the per-row pass 2, 2 = float32 filter with
+ *       the tiled pass 2, 3 = filter abandoned for the exact pass (non-finite input or too many candidates)
+ *   [5] SMs of the device
+ * All zeros before the thread's first linkage.  Diagnostics only: needs no device and changes no result. */
+void fa_ahc_last_placement(int32_t *out6);
+
 /* Swift-side dendrogram cut + relabel on a SciPy-format linkage Z [(count-1) x 4]. */
 fa_status fa_dendrogram_cut(const double *Z, size_t count, double threshold, int32_t *labels);
 

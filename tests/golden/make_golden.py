@@ -14,6 +14,12 @@
               where the reference cannot be compiled.  Record them by running the whole suite (GPU tests included)
               and smoke() with oracle/_ref built and FA_ORACLE_RECORD_REF=<dir>, then
               `python tests/golden/make_golden.py ref_linkage <dir>`.
+* ahc_placements.json  the reference's status and dendrogram SHA-256, and the SHA-256 of the labels cut at 0.6, for the
+              linkage problems that reach each placement of the CUDA merge loop and initial pass (PLACEMENT_CASES), plus
+              the SHA-256 of the final pipeline labels (oracle.diarize_cluster) of the batch sets (BATCH_SETS).  Inputs
+              are regenerated from seeds; recording also checks that the restatement reproduces every dendrogram.
+              `python tests/golden/make_golden.py placements` regenerates only this file (several CPU-minutes per
+              large case; the cases run in parallel).
 * mel_*.npz   log-mel of the reference's own test signal (SortformerStreamingMelTests.swift:17-25 shape) from the
               oracle restatement: the reference has no golden mel values and no Swift toolchain exists here, so
               these pin the oracle against silent drift, not against Apple's vDSP.
@@ -72,10 +78,100 @@ def pack_ref_linkage(src):
     print(f"{len(records)} reference records in {path}")
 
 
+# ---- linkage placements (tests/test_gpu_cluster_config_space.py) -----------------------------------------------------
+# name: (N, D, kind, seed).  kinds: "speaker" = L2-normalised synthetic speaker embeddings (8 speakers); "gauss" = raw
+# standard normal rows; "eighths" = standard normal rounded to multiples of 1/8 (exact in binary, so equal distances are
+# exact ties); "dupes" = 20 distinct standard normal rows, 200 copies each, shuffled.
+PLACEMENT_CASES = {
+    "l3_11376x32": (11376, 32, "speaker", 101),
+    "l2_11377x32": (11377, 32, "speaker", 102),
+    "l2_14176x32": (14176, 32, "speaker", 103),
+    "l1_14177x32": (14177, 32, "speaker", 104),
+    "l2_ties_12000x8": (12000, 8, "eighths", 105),
+    "l1_resident_15000x256": (15000, 256, "speaker", 106),
+    "l1_streamed_17000x256": (17000, 256, "speaker", 107),
+    "l1_full_18800x64": (18800, 64, "speaker", 108),
+    "l1_18808x8": (18808, 8, "speaker", 117),
+    "l0_resident_18809x8": (18809, 8, "speaker", 118),
+    "l0_streamed_19000x64": (19000, 64, "speaker", 109),
+    "l0_tiles_33000x16": (33000, 16, "speaker", 110),
+    "tiles_2050x1600": (2050, 1600, "speaker", 111),
+    "pad_2048x1": (2048, 1, "gauss", 112),
+    "pad_3000x3": (3000, 3, "gauss", 113),
+    "pad_2500x300": (2500, 300, "speaker", 114),
+    "pad_4097x257": (4097, 257, "speaker", 115),
+    "overflow_4000x8": (4000, 8, "dupes", 116),
+}
+# batches for fa_diarize_cluster_batch: lists of (N, seed) at D = 256; the 17 000-row set is l1_streamed_17000x256's
+BATCH_SETS = {
+    "four_lanes": [(17000, 107), (400, 201), (400, 202), (400, 203)],
+    "two_lanes": [(6000, 204), (6000, 205), (6000, 206)],
+}
+
+
+def placement_input(n, d, kind, seed):
+    """(linkage input [n x d] float64, the float32 embeddings it was normalised from or None)."""
+    if kind == "speaker":
+        emb, _ = synth.speaker_embeddings(n, d, 8, seed=seed)
+        return O.l2_normalize_rows(emb.astype(np.float64)), emb
+    rng = np.random.default_rng(seed)
+    if kind == "gauss":
+        return rng.standard_normal((n, d)), None
+    if kind == "eighths":
+        return np.round(rng.standard_normal((n, d)) * 8.0) / 8.0, None
+    assert kind == "dupes" and n % 20 == 0
+    return np.repeat(rng.standard_normal((20, d)), n // 20, axis=0)[rng.permutation(n)], None
+
+
+def batch_set(n, seed):
+    """(embeddings float32 [n x 256], rho [n x 128], psi [128]) of one batch set."""
+    emb, _ = synth.speaker_embeddings(n, 256, 8, seed=seed)
+    rho, psi = synth.synthetic_plda(emb)
+    return emb, rho, psi
+
+
+def _sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def _record_linkage(name):
+    n, d, kind, seed = PLACEMENT_CASES[name]
+    x, _ = placement_input(n, d, kind, seed)
+    st, z = O.centroid_linkage(x, use_ref=True)
+    st2, z2 = O.centroid_linkage(x)
+    assert st == st2 == 0 and np.array_equal(z, z2), f"{name}: the restatement differs from the reference"
+    return name, {"n": n, "d": d, "kind": kind, "seed": seed, "status": st, "z_sha256": _sha(z),
+                  "labels_sha256": _sha(O.dendrogram_cut(z, n, 0.6))}
+
+
+def _record_pipeline(key):
+    n, seed = key
+    emb, rho, psi = batch_set(n, seed)
+    return f"{n}_seed{seed}", {"n": n, "seed": seed,
+                               "final_labels_sha256": _sha(O.diarize_cluster(emb, rho, psi, use_ref=True).labels)}
+
+
+def placements():
+    from concurrent.futures import ProcessPoolExecutor
+    jobs = sorted({s for sets in BATCH_SETS.values() for s in sets}, key=lambda s: -s[0])
+    names = sorted(PLACEMENT_CASES, key=lambda k: -PLACEMENT_CASES[k][0] * PLACEMENT_CASES[k][1] ** 0.5)
+    with ProcessPoolExecutor(os.cpu_count()) as pool:
+        pipes = [pool.submit(_record_pipeline, k) for k in jobs]
+        links = [pool.submit(_record_linkage, k) for k in names]
+        out = {"linkage": dict(f.result() for f in links), "pipelines": dict(f.result() for f in pipes)}
+    with open(os.path.join(HERE, "ahc_placements.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print(f"ahc_placements.json written: {len(out['linkage'])} linkages, {len(out['pipelines'])} pipelines")
+
+
 def main():
     O.build()
     if len(sys.argv) > 1 and sys.argv[1] == "next":
         return next_rows()
+    if len(sys.argv) > 1 and sys.argv[1] == "placements":
+        assert O.ref_available(), "oracle/_ref/liboracle_fc.so missing: run `make -C oracle ref` where the reference exists"
+        return placements()
     if len(sys.argv) > 2 and sys.argv[1] == "ref_linkage":
         return pack_ref_linkage(sys.argv[2])
     assert O.ref_available(), "oracle/_ref/liboracle_fc.so missing: run `make -C oracle ref` where /root/reference exists"

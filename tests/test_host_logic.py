@@ -47,6 +47,23 @@ def test_library_exports_every_declared_symbol(lib):
     assert all(s.startswith("fa_") or s.startswith("fastcluster_") for s in exported), sorted(exported)[:10]
 
 
+def test_ahc_placement_diagnostic_is_zero_before_any_linkage(lib):
+    """fa_ahc_last_placement reports the calling thread's last linkage: a fresh thread sees zeros, without a device."""
+    import threading
+    seen = []
+
+    def read():
+        out = np.full(6, -1, np.int32)
+        lib.fa_ahc_last_placement(out.ctypes.data)
+        seen.append(out.tolist())
+
+    t = threading.Thread(target=read)
+    t.start()
+    t.join()
+    assert seen == [[0] * 6]
+    lib.fa_ahc_last_placement(None)   # a null output is ignored
+
+
 def test_reference_argument_contract_needs_no_device(lib):
     """FastClusterWrapper.cpp:203-223 — these statuses are decided before any clustering work."""
     f = lib.fastcluster_compute_centroid_linkage
